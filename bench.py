@@ -16,6 +16,12 @@ One "step" = one decode step (one token for the whole batch) through all 32 laye
              cores: real full-depth decode steps, as many as fit a 25 s box.  Host threads = the fastest count of a short
              sweep up to the CPUs the process may use (affinity mask capped by the cgroup quota), see calibrate_threads.
 N GPUs = tensor parallel over N ranks (the reference's scheme; strong scaling: one model, one token stream).
+
+--dump-outputs DIR writes what the last timed step of `value` computed, as a caller of that step receives it:
+  DIR/logits.npy      float32 [bsz, vocab]   the step's logits
+  DIR/next_token.npy  float64 [bsz]          the greedy token the step fed back (argmax of those logits)
+Weights, KV cache and the first token are drawn from fixed seeds, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -345,6 +351,14 @@ def tp_warmup_verdict(tokens, ar_err):
     return bool(torch.equal(lo, hi)), int(bad.item())
 
 
+def dump_outputs(out_dir, logits, tokens):
+    """The last timed step's results as DIR/<name>.npy (float32 / float64: 128 KB at the headline workload)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), logits.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "next_token.npy"), tokens.cpu().numpy().astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -356,7 +370,13 @@ def main():
     ap.add_argument("--no-pdl", action="store_true")
     ap.add_argument("--bits", type=int, default=4)
     ap.add_argument("--group-size", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's logits and next token as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU engine (--impl b200)")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -455,6 +475,8 @@ def main():
             torch.cuda.synchronize()
             _log(f"step {i} ok")
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.greedy_logits[:BSZ], eng.tokens[:BSZ])
     total_ms = ev[0].elapsed_time(ev[K])
     per_step = sorted(ev[i].elapsed_time(ev[i + 1]) for i in range(K))
     clk = clocks.stop() if clocks else None

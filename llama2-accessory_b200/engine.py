@@ -787,11 +787,13 @@ class DecodeEngine:
     def capture_greedy_loop(self, bsz: int):
         """One CUDA graph = one full greedy decode step with everything resident on the device:
         step(tokens, pos) -> argmax -> tokens, pos += 1   (meta.py:434-448 without the per-token host sync).
-        Returns (graph, launches_per_step). Set self.tokens[:bsz] / self.pos[:bsz] before the first replay."""
+        Returns (graph, launches_per_step). Set self.tokens[:bsz] / self.pos[:bsz] before the first replay.
+        After a replay, self.greedy_logits holds that step's fp32 logits [bsz, vocab] (the graph's static output)."""
         def body():
             logits = self._step(bsz, 1, self.cache_seq)
             ops.argmax(logits.contiguous(), self.tokens, bsz, logits.shape[-1])
             ops.advance_pos(self.pos, bsz, 1)
+            return logits
         keep_tok, keep_pos = self.tokens.clone(), self.pos.clone()
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
@@ -804,7 +806,7 @@ class DecodeEngine:
         g = torch.cuda.CUDAGraph()
         n0 = ops.launch_count
         with torch.cuda.graph(g):
-            body()
+            self.greedy_logits = body()
         return g, ops.launch_count - n0
 
     @torch.inference_mode()

@@ -62,10 +62,10 @@ def expand_kv(x, n_rep):
     return x[:, :, :, None, :].expand(b, s, h, n_rep, d).reshape(b, s, h * n_rep, d)
 
 
-def causal_mask(q_len, kv_len):
+def causal_mask(q_len, kv_len, device=None):
     """llama.py:220-224: right-aligned boolean mask."""
-    qi = torch.arange(q_len) - q_len
-    ki = torch.arange(kv_len) - kv_len
+    qi = torch.arange(q_len, device=device) - q_len
+    ki = torch.arange(kv_len, device=device) - kv_len
     return qi.view(-1, 1) >= ki.view(1, -1)
 
 
@@ -81,8 +81,9 @@ class PortModel:
         self.eps = a.get("norm_eps", 1e-5)
         self.max_seq_len = a.get("max_seq_len", 2048)
         theta = a.get("rope_theta", 10000.0 if kind == "llama" else 1000000.0)
-        self.freqs_cis = precompute_freqs_cis(self.hd, self.max_seq_len * 2, theta, a.get("rope_scaling"))
         self.sd = {k: v.to(dtype) for k, v in sd.items()}
+        self.device = next(iter(self.sd.values())).device  # the model runs where its weights are (CPU or GPU)
+        self.freqs_cis = precompute_freqs_cis(self.hd, self.max_seq_len * 2, theta, a.get("rope_scaling")).to(self.device)
         assert self.H % tp == 0 and self.Hkv % tp == 0
         self.k_cache = self.v_cache = None
         if kind == "mixtral":
@@ -106,8 +107,8 @@ class PortModel:
     def alloc_cache(self, bsz):
         shape = (bsz, self.max_seq_len, self.Hkv, self.hd)
         if self.k_cache is None or self.k_cache[0].shape != shape:
-            self.k_cache = [torch.zeros(shape, dtype=self.dtype) for _ in range(self.L)]
-            self.v_cache = [torch.zeros(shape, dtype=self.dtype) for _ in range(self.L)]
+            self.k_cache = [torch.zeros(shape, dtype=self.dtype, device=self.device) for _ in range(self.L)]
+            self.v_cache = [torch.zeros(shape, dtype=self.dtype, device=self.device) for _ in range(self.L)]
 
     # -- blocks ---------------------------------------------------------------------------
     def attention(self, i, x, start_pos, fc, causal):
@@ -125,7 +126,7 @@ class PortModel:
         n_rep = self.H // self.Hkv
         kk = expand_kv(keys, n_rep).transpose(1, 2)
         vv = expand_kv(vals, n_rep).transpose(1, 2)
-        mask = causal_mask(S, keys.shape[1]) if causal else None
+        mask = causal_mask(S, keys.shape[1], x.device) if causal else None
         o = F.scaled_dot_product_attention(q.transpose(1, 2), kk, vv, dropout_p=0.0, attn_mask=mask)
         o = o.transpose(1, 2).contiguous().view(B, S, -1)
         wo = self._w(p + "wo.weight")

@@ -8,6 +8,7 @@ fp16.  RMSNorm weights are 1 + small deterministic perturbation when `perturb_no
 exercise the gamma multiply), else exactly 1 as in components.py:26.
 Master (TP=1) tensors are generated once; shards are slices of them.
 """
+import hashlib
 import math
 import zlib
 
@@ -129,3 +130,9 @@ def shard_state_dict(sd: dict, rank: int, world: int, kind: str = "llama"):
         else:
             out[k] = v
     return out
+
+
+def tensor_digest(t: torch.Tensor) -> dict:
+    """dtype, shape and sha256 of the bytes: a stored stand-in for a tensor that a test compares with torch.equal."""
+    raw = t.detach().cpu().contiguous().reshape(-1).view(torch.uint8).numpy().tobytes()
+    return {"dtype": str(t.dtype), "shape": list(t.shape), "sha256": hashlib.sha256(raw).hexdigest()}

@@ -19,7 +19,7 @@ from llama2_accessory_b200 import checkpoint as ck
 from llama2_accessory_b200 import quant
 from llama2_accessory_b200.engine import DecodeEngine, EngineConfig
 from oracle import cases, omniquant
-from oracle.weights import shard_state_dict
+from oracle.weights import shard_state_dict, tensor_digest
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -225,35 +225,27 @@ def test_checkpoint_folder_to_engine_and_packed_round_trip(tmp_path, kind, bits,
 
 
 def test_merge_and_inference_agree_with_the_reference_loader(tmp_path):
-    """The UNMODIFIED accessory/util/tensor_parallel.py (imported in the build container, world size 1 shim) reads the
-    same folders: format inference and the merged TP = 1 state dict must agree tensor for tensor."""
-    from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib
-    ref_import.load("llama")
-    tp = importlib.import_module("accessory.util.tensor_parallel")
+    """The UNMODIFIED accessory/util/tensor_parallel.py read the same folders (tests/golden/reference_tp_loader.json, made
+    by oracle/make_golden_loader.py): format inference, shard file names and the merged TP = 1 state dict must agree tensor
+    for tensor, the merged dict must fit the reference Transformer's parameter names, and the same malformed folders are
+    refused."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_tp_loader.json")) as f:
+        gold = json.load(f)
     args, sd = _master("llama")
-    model = ref_import.build_reference_model("llama", dict(args), sd, torch.float16)
-    holder = torch.nn.Module()
-    holder.llma = model
-    for fmt in ("consolidated", "meta_ori"):
+    ref_keys = set(gold["model_keys"])
+    for fmt, g in gold["formats"].items():
         d = str(tmp_path / fmt)
         ck.save_tensor_parallel_shards(sd, d, 2, fmt)
-        assert tuple(tp.infer_checkpoint_format_and_mp_size(d)) == ck.infer_checkpoint_format_and_mp_size(d) == (fmt, 2)
-        assert tp.get_tensor_parallel_shards_file_name(fmt, 2) == ck.get_tensor_parallel_shards_file_name(fmt, 2)
-        import contextlib
-        import io
-        with contextlib.redirect_stdout(io.StringIO()):
-            ref_sd = tp.load_tensor_parallel_model_state_dict(holder, d, fmt)
+        assert ck.infer_checkpoint_format_and_mp_size(d) == tuple(g["inferred"]) == (fmt, 2)
+        assert ck.get_tensor_parallel_shards_file_name(fmt, 2) == g["shard_file_names"]
         mine = ck.load_tensor_parallel_state_dict(d, 0, 1, fmt)
-        assert set(ref_sd) == set(mine)
-        for k in ref_sd:
-            assert torch.equal(ref_sd[k], mine[k]), k
+        assert set(g["merged"]) == set(mine)
+        for k in mine:
+            assert tensor_digest(mine[k]) == g["merged"][k], k
         # and it loads into the reference model without missing / unexpected weights
-        res = holder.load_state_dict(ref_sd, strict=False)
-        assert not res.unexpected_keys and all("clip" in k or "rope" in k or "freqs" in k for k in res.missing_keys)
-    for bad in ("empty", "mixed"):
+        assert set(mine) <= ref_keys and all("clip" in k or "rope" in k or "freqs" in k for k in ref_keys - set(mine))
+    assert gold["refused"] == {"empty": "NotImplementedError", "mixed": "NotImplementedError"}
+    for bad in gold["refused"]:
         d = tmp_path / bad
         d.mkdir()
         if bad == "mixed":
@@ -261,8 +253,6 @@ def test_merge_and_inference_agree_with_the_reference_loader(tmp_path):
             ck.save_tensor_parallel_shards(sd, str(d), 1, "meta_ori")
         else:
             (d / "x.txt").write_text("x")
-        with pytest.raises(NotImplementedError):
-            tp.infer_checkpoint_format_and_mp_size(str(d))
         with pytest.raises(NotImplementedError):
             ck.infer_checkpoint_format_and_mp_size(str(d))
 

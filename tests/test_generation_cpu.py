@@ -24,8 +24,9 @@ GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "
 def model():
     args = dict(cases.TINY_LLAMA)
     port = PortModel("llama", args, cases.master_state_dict("llama", args), dtype=torch.float32)
+    # parameters(): the loop keeps its token buffers where the model's weights are (the CPU), on a GPU host as well
     return types.SimpleNamespace(args=types.SimpleNamespace(max_seq_len=args["max_seq_len"], max_batch_size=args["max_batch_size"]),
-                                 forward_inference=port.forward_inference)
+                                 forward_inference=port.forward_inference, parameters=lambda: iter(port.sd.values()))
 
 
 def _argmax(logits, temperature, top_p):
@@ -53,7 +54,7 @@ def test_generate_matches_reference_loop_mixtral():
     args = dict(cases.TINY_MIXTRAL)
     port = PortModel("mixtral", args, cases.master_state_dict("mixtral", args), dtype=torch.float32)
     m = types.SimpleNamespace(args=types.SimpleNamespace(max_seq_len=args["max_seq_len"], max_batch_size=args["max_batch_size"]),
-                              forward_inference=port.forward_inference)
+                              forward_inference=port.forward_inference, parameters=lambda: iter(port.sd.values()))
     for case in GOLD["mixtral_cases"]:
         tok = ToyTokenizer(args["vocab_size"], case["eos_id"])
         assert generation.generate(m, tok, list(GOLD["prompts"]), select=_argmax, device_loop=False, **case["kwargs"]) == case["texts"]

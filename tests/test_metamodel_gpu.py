@@ -1,19 +1,16 @@
-"""GPU: the UNMODIFIED reference `MetaModel` (accessory/model/meta.py, imported byte-for-byte from /root/reference or its
-staged copy oracle/_ref) constructed with ``llama_type="llama_b200"`` and driven through its own ``generate()``.
+"""GPU: the UNMODIFIED reference `MetaModel` (accessory/model/meta.py) constructed with ``llama_type="llama_b200"`` and
+driven through its own ``generate()`` -- the integration level 3 of INTEGRATION.md -- against this package's statement of
+that loop over the same engine.
 
-This is the integration level 3 of INTEGRATION.md executed end to end: `MetaModel.__init__` (meta.py:20-78) resolves
-``accessory.model.LLM.llama_b200`` with importlib (meta.py:29), reads the JSON config into our ``ModelArgs``, builds our
-``Transformer``; a checkpoint-shaped state dict is loaded into ``model.llma``; ``MetaModel.generate`` (meta.py:372-468)
-then calls ``self.llma.forward_inference`` once per token -- every one of those calls runs in libb200decode.so.
-
-The modules meta.py imports but this path never touches (util.misc / util.tensor_parallel / model.tokenizer) are stubbed
-as in oracle/make_golden_generate.py; the tokenizer is the toy whitespace tokenizer the generate-loop goldens use.
+`MetaModel.__init__` (meta.py:20-78) resolves ``accessory.model.LLM.llama_b200``, reads the JSON config into our
+``ModelArgs`` (max_batch_size 32, vocab size from the tokenizer) and builds our ``Transformer``; a checkpoint-shaped state
+dict is loaded into it; ``MetaModel.generate`` (meta.py:372-468) then calls ``forward_inference`` once per token, every one
+of those calls running in libb200decode.so.  What it returned on a B200 is stored in tests/golden/metamodel_generate.json
+(oracle/make_golden_metamodel.py); here the same ``Transformer`` is built from the same config, and generation.generate /
+stream_generate must return those texts.  The tokenizer is the toy whitespace tokenizer the generate-loop goldens use.
 """
-import importlib
 import json
 import os
-import sys
-import types
 
 import pytest
 import torch
@@ -23,44 +20,19 @@ pytestmark = pytest.mark.gpu
 import llama2_accessory_b200 as pkg  # noqa: E402
 from llama2_accessory_b200 import generation  # noqa: E402
 from llama2_accessory_b200.model import llama_b200  # noqa: E402
-from oracle import cases, ref_import  # noqa: E402
+from oracle import cases  # noqa: E402
 from oracle.toy_tokenizer import ToyTokenizer  # noqa: E402
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "generate.json")
+GOLD_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLD = os.path.join(GOLD_DIR, "generate.json")
 PROMPTS = ["the quick brown fox", "hello world", "a b c d e f g"]
 
 
-class _PathTokenizer(ToyTokenizer):
-    """accessory/model/tokenizer.py::Tokenizer(model_path=...) stand-in: 'toy:<n_words>:<eos_id>'."""
-
-    def __init__(self, model_path):
-        _, n, eos = model_path.split(":")
-        super().__init__(int(n), int(eos))
-
-
-def _import_meta():
-    if not ref_import.available():
-        pytest.skip("reference tree not staged (oracle/_ref)")
-    ref_import.load("llama")  # registers the accessory namespace packages + the fairscale shim
-    stubs = (("accessory.util.misc", {"mark_mp_params": lambda model: None}),
-             ("accessory.util.tensor_parallel", {}),
-             ("accessory.model.tokenizer", {"Tokenizer": _PathTokenizer, "probe_tokenizer_path_from_pretrained": None}))
-    for name, attrs in stubs:
-        m = sys.modules.get(name)
-        if m is None:
-            m = types.ModuleType(name)
-            sys.modules[name] = m
-            parent, leaf = name.rsplit(".", 1)
-            setattr(sys.modules[parent], leaf, m)
-        for k, v in attrs.items():
-            setattr(m, k, v)
-    # the two-line plug-in file of INTEGRATION.md section 3 (accessory/model/LLM/llama_b200.py), registered in memory
-    plug = types.ModuleType("accessory.model.LLM.llama_b200")
-    plug.ModelArgs, plug.Transformer = llama_b200.ModelArgs, llama_b200.Transformer
-    sys.modules["accessory.model.LLM.llama_b200"] = plug
-    meta = importlib.import_module("accessory.model.meta")
-    meta.Tokenizer = _PathTokenizer  # in case meta.py was imported earlier in this process with another stub
-    return meta
+def _meta_gold():
+    with open(os.path.join(GOLD_DIR, "metamodel_generate.json")) as f:
+        g = json.load(f)
+    assert g["prompts"] == PROMPTS
+    return g
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -68,62 +40,65 @@ def _built():
     pkg.build()
 
 
-def _metamodel(meta, tmp_path, wbits, eos_id=2):
+def _metamodel(wbits, eos_id=2):
+    """The Transformer and tokenizer MetaModel('llama_b200', <config with wbits>, 'toy:<vocab>:<eos>') holds (meta.py:33-56)."""
     args = dict(cases.TINY_LLAMA)
     cfg = {k: v for k, v in args.items() if k not in ("vocab_size", "max_seq_len", "max_batch_size")}
     cfg["wbits"] = wbits
-    p = tmp_path / f"config_w{wbits}.json"
-    p.write_text(json.dumps(cfg))
+    tok = ToyTokenizer(args["vocab_size"], eos_id)
+    margs = llama_b200.ModelArgs(**cfg, max_seq_len=args["max_seq_len"], max_batch_size=32,
+                                 vocab_size=tok.n_words)
     old = torch.get_default_dtype()
     torch.set_default_dtype(torch.float16)
     try:
         with torch.device("cuda"):
-            model = meta.MetaModel("llama_b200", str(p), f"toy:{args['vocab_size']}:{eos_id}", with_visual=False,
-                                   max_seq_len=args["max_seq_len"])
+            model = llama_b200.Transformer(margs, with_visual=False)
     finally:
         torch.set_default_dtype(old)
-    assert type(model.llma) is llama_b200.Transformer and model.llma.args.max_batch_size == 32
+    assert model.args.max_batch_size == 32
     sd = cases.master_state_dict("llama", args)
-    missing, unexpected = model.load_state_dict({"llma." + k: v.cuda() for k, v in sd.items()}, strict=False)
+    missing, unexpected = model.load_state_dict({k: v.cuda() for k, v in sd.items()}, strict=False)
     assert not missing and not unexpected, (missing, unexpected)
-    return model.eval()
+    return model.eval(), tok
 
 
-def test_unmodified_metamodel_generate_runs_on_the_b200_engine(tmp_path):
-    meta = _import_meta()
-    model = _metamodel(meta, tmp_path, wbits=4)
-    texts = model.generate(list(PROMPTS), max_gen_len=6)
-    assert model.llma.engine is not None and model.llma.engine.cfg.bits == 4  # forward_inference built the packed engine
+def test_generate_reproduces_the_unmodified_metamodel_on_the_b200_engine():
+    g = _meta_gold()["w4"]
+    model, tok = _metamodel(wbits=4)
+    texts = generation.generate(model, tok, list(PROMPTS), max_gen_len=6, device_loop=False)
+    assert model.engine is not None and model.engine.cfg.bits == 4  # forward_inference built the packed engine
+    assert texts == g["greedy"], (texts, g["greedy"])
     # the loop runs to max(prompt length) + max_gen_len for every row (meta.py:415-433): shorter prompts generate more tokens
-    plens = [len(model.tokenizer.encode(x, bos=True, eos=False)) for x in PROMPTS]
+    plens = [len(tok.encode(x, bos=True, eos=False)) for x in PROMPTS]
     assert [len(t.split()) for t in texts] == [max(plens) + 6 - n for n in plens], texts
-    tok = model.tokenizer
-    # same tokens as this repo's statement of the loop (host and device drivers) over the same engine
-    assert generation.generate(model.llma, tok, list(PROMPTS), max_gen_len=6, device_loop=False) == texts
-    assert generation.generate(model.llma, tok, list(PROMPTS), max_gen_len=6, device_loop=True) == texts
+    # same tokens from the device-resident driver of the loop over the same engine
+    assert generation.generate(model, tok, list(PROMPTS), max_gen_len=6, device_loop=True) == texts
     # eos / stop-symbol handling of the reference loop over our logits
     row0 = [int(w[1:]) for w in texts[0].split()]
-    model.tokenizer.eos_id = row0[2]
-    cut = model.generate(list(PROMPTS), max_gen_len=6)
+    assert g["eos_id_cut"] == row0[2]
+    tok.eos_id = row0[2]
+    cut = generation.generate(model, tok, list(PROMPTS), max_gen_len=6, device_loop=False)
     first = row0.index(row0[2])  # the reference stops a row at the FIRST occurrence of eos among its generated tokens
-    assert cut[0] == " ".join(texts[0].split()[:first]), (cut, texts)
-    assert cut == generation.generate(model.llma, model.tokenizer, list(PROMPTS), max_gen_len=6, device_loop=False)
-    model.tokenizer.eos_id = 2
+    assert cut == g["eos_cut"] and cut[0] == " ".join(texts[0].split()[:first]), (cut, g["eos_cut"], texts)
+    tok.eos_id = 2
     stops = (f"w{row0[1]} w{row0[2]}",)
-    stop = model.generate(list(PROMPTS), max_gen_len=6, additional_stop_symbols=stops)
-    assert stop == generation.generate(model.llma, model.tokenizer, list(PROMPTS), max_gen_len=6, additional_stop_symbols=stops,
-                                       device_loop=False)
+    assert list(stops) == g["stop_symbols"]
+    stop = generation.generate(model, tok, list(PROMPTS), max_gen_len=6, additional_stop_symbols=stops, device_loop=False)
+    assert stop == g["stop"], (stop, g["stop"])
     assert len(stop[0].split()) < len(texts[0].split()), (stop, texts)
-    ys = list(model.stream_generate(PROMPTS[0], max_gen_len=5))
-    assert ys[-1]["end_of_content"] and ys[-1]["text"] == model.generate([PROMPTS[0]], max_gen_len=5)[0]
+    ys = list(generation.stream_generate(model, tok, PROMPTS[0], max_gen_len=5))
+    assert ys == g["stream_prompt0"], (ys, g["stream_prompt0"])
+    single = generation.generate(model, tok, [PROMPTS[0]], max_gen_len=5)
+    assert single == g["single_prompt0"] and ys[-1]["end_of_content"] and ys[-1]["text"] == single[0]
 
 
-def test_metamodel_fp16_engine_against_the_reference_goldens(tmp_path):
+def test_metamodel_fp16_engine_against_the_reference_goldens():
     """wbits = 16: the same weights the fp32 goldens of the unmodified reference model were generated from
-    (tests/golden/generate.json); fp16 logits can flip a near-tie, so agreement is counted, not demanded token for token."""
-    meta = _import_meta()
-    model = _metamodel(meta, tmp_path, wbits=16)
-    texts = model.generate(list(PROMPTS), max_gen_len=6)
+    (tests/golden/generate.json); fp16 logits can flip a near-tie, so agreement is counted, not demanded token for token.
+    The texts are those the unmodified MetaModel returned over the fp16 engine."""
+    model, tok = _metamodel(wbits=16)
+    texts = generation.generate(model, tok, list(PROMPTS), max_gen_len=6)
+    assert texts == _meta_gold()["w16"]["greedy"], texts
     gold = next(c for c in json.load(open(GOLD))["cases"] if c["name"] == "greedy")["texts"]
     first = sum(a.split()[0] == b.split()[0] for a, b in zip(texts, gold))
     n_tok = sum(len(b.split()) for b in gold)
