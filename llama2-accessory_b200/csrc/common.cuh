@@ -77,20 +77,25 @@ __device__ __forceinline__ void l2_prefetch(const void* src, uint32_t bytes) {
 // L2 prefetch of the head of the NEXT kernel's weight stream.  n_tiles > 0: the next GEMV (grid next_grid) gives CTA r
 // the contiguous tiles [n_tiles*r/next_grid, n_tiles*(r+1)/next_grid); the first `window` bytes of every region are
 // prefetched, one region per calling CTA.  n_tiles == 0: [0, total) as one range, split over the calling CTAs.
+// The loops stay rolled: one thread runs them once per launch, and unrolled copies only take instruction-cache space from
+// the warps that share the SM.
 __device__ __forceinline__ void prefetch_next_stream(const uint8_t* base, int total, int n_tiles, int next_grid,
                                                      int window, int cta, int n_cta) {
   constexpr uint32_t piece = 16384;
   if (n_tiles > 0 && next_grid > 0) {
     const int tile_bytes = total / n_tiles;
+#pragma unroll 1
     for (int r = cta; r < next_grid; r += n_cta) {
       const long long t0 = ((long long)n_tiles * r) / next_grid, t1 = ((long long)n_tiles * (r + 1)) / next_grid;
       const long long bytes = min((t1 - t0) * (long long)tile_bytes, (long long)window);
       const uint8_t* src = base + t0 * tile_bytes;
+#pragma unroll 1
       for (long long off = 0; off < bytes; off += piece)
         l2_prefetch(src + off, (uint32_t)min((long long)piece, bytes - off) & ~15u);
     }
   } else {
     const int n_piece = (total + (int)piece - 1) / (int)piece;
+#pragma unroll 1
     for (int i = cta; i < n_piece; i += n_cta) {
       const uint32_t off = (uint32_t)i * piece;
       const uint32_t len = min(piece, (uint32_t)total - off) & ~15u;

@@ -39,8 +39,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv1_kernel(const __grid_constan
   sm.empty = sm.full + p.stages;
   sm.red_full = sm.empty + p.stages;
   sm.red_empty = sm.red_full + 2;
-  uint64_t* x_ready = sm.red_empty + 2;  // the 16 MMA warps arrive once their slice of x is staged (+ 1 word of padding)
-  sm.red = reinterpret_cast<int*>(x_ready + 2);
+  sm.red = reinterpret_cast<int*>(sm.red_empty + 2);
   sm.scratch = reinterpret_cast<float*>(sm.red + 2 * kConsumerWarps * 128);
   sm.xq = reinterpret_cast<uint8_t*>(sm.scratch + 32);
   sm.szr = sm.xq + (size_t)kPlanes * ((((p.K + 127) >> 7) << 7) + 64);  // GROUPED only (not allocated otherwise)
@@ -56,7 +55,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemv1_kernel(const __grid_constan
       mbar_init(&sm.red_full[b], kConsumerWarps);
       mbar_init(&sm.red_empty[b], kEpiWarps);
     }
-    mbar_init(x_ready, kConsumerWarps);
     fence_mbar_init();
   }
   if (tid < 256) sm.red[tid] = 0;  // the two [16][8] blocks the MMA warps add their integer partial sums into
@@ -70,61 +68,16 @@ __global__ void __launch_bounds__(kThreads, 1) gemv1_kernel(const __grid_constan
     // ---------------- producer: weight stream, independent of any earlier kernel ----------------
     if (lane == 0) {
       if (cta == 0 && p.const_pf && p.const_pf_bytes > 0) l2_prefetch(p.const_pf, (uint32_t)p.const_pf_bytes & ~15u);
-      // L2 prefetches of this launch.  pf_early: issued when the ring is full for the first time, i.e. while the
-      // consumers still wait for the previous kernel and the HBM pipe would otherwise idle; else after the last own slot.
-      auto kv_prefetch = [&](bool wait) {
-        // the attention kernel that follows streams K/V rows [0, pos] of every kv head.  pos[] is written by a kernel
-        // outside the programmatic chain; an early (pre-dependency) read can at worst see the previous step's value,
-        // which only shortens the hint by one row -- the value is clamped to the cache, the prefetch is a hint.
-        if (wait) pdl_wait();
-        const int kv_len = min(max(p.pos[0], 0) + 1, p.cache_seq);
-        const int brow = p.t_base / p.tokens_per_seq;
-        const uint32_t k_bytes = (uint32_t)kv_len * 256u, v_bytes = (uint32_t)((kv_len + 31) >> 5) * 8192u;
-        constexpr uint32_t piece = 16384;
-        const int kp = (int)((k_bytes + piece - 1) / piece), vp = (int)((v_bytes + piece - 1) / piece);
-        const int total = p.hkv * (kp + vp);
-        for (int i = cta; i < total; i += n_cta) {
-          const int head = i / (kp + vp), j = i % (kp + vp);
-          const size_t base = ((size_t)brow * p.hkv + head) * p.cache_seq * 128;  // halfs, same for K and V
-          if (j < kp) {
-            const uint32_t off = (uint32_t)j * piece;
-            l2_prefetch(reinterpret_cast<const uint8_t*>(p.kcache + base) + off, min(piece, k_bytes - off));
-          } else {
-            const uint32_t off = (uint32_t)(j - kp) * piece;
-            l2_prefetch(reinterpret_cast<const uint8_t*>(p.vtcache + base) + off, min(piece, v_bytes - off));
-          }
-        }
-      };
       const int tile_begin = (int)(((long long)p.n_tiles * cta) / n_cta);
       const int tile_end = (int)(((long long)p.n_tiles * (cta + 1)) / n_cta);
       const int slots_per_tile = (p.KB + kSlotBlocks - 1) / kSlotBlocks;
-      const uint8_t* region = p.qw + (size_t)tile_begin * p.KB * 512;
-      const long long region_bytes = (long long)(tile_end - tile_begin) * p.KB * 512;
-      bool early_done = false;
-      auto early = [&](long long issued_bytes) {
-        early_done = true;
-        if (p.self_pf_bytes > 0) {
-          const long long end = min(region_bytes, issued_bytes + (long long)p.self_pf_bytes);
-          for (long long off = issued_bytes; off < end; off += 16384)
-            l2_prefetch(region + off, (uint32_t)min(16384ll, end - off));
-        }
-        if (p.pf_early) {
-          if (p.next_w && p.next_bytes > 0)
-            prefetch_next_stream(p.next_w, p.next_bytes, p.next_tiles, p.next_grid, p.next_window, cta, n_cta);
-          if (EPI == B200_EPI_QKV && p.prefetch_kv) kv_prefetch(false);
-        }
-      };
-      int stage = 0, issued = 0;
+      int stage = 0;
       uint32_t par = 0;
-      long long issued_bytes = 0;
       const uint64_t pol_ef = l2_policy_evict_first();
       for (int tile = tile_begin; tile < tile_end; ++tile) {
         const uint8_t* src = p.qw + (size_t)tile * p.KB * 512;
+#pragma unroll 1
         for (int s = 0; s < slots_per_tile; ++s) {
-          if (!early_done && issued == p.stages) early(issued_bytes);  // the next wait would block: the ring is full
-          // experiment knob: hold the weight stream after `hold_slots` slots until x is staged, so that the activation
-          // loads of the MMA warps do not queue behind this SM's own bulk copies
-          if (p.hold_slots > 0 && issued == p.hold_slots) mbar_wait(x_ready, 0);
           mbar_wait(&sm.empty[stage], par ^ 1);
           const int nblk = min(kSlotBlocks, p.KB - s * kSlotBlocks);
           const uint32_t bytes = (uint32_t)nblk * 512u;
@@ -140,18 +93,31 @@ __global__ void __launch_bounds__(kThreads, 1) gemv1_kernel(const __grid_constan
           }
           if (p.stream_ef) bulk_g2s_hint(sm.ring + (size_t)stage * kSlotBytes, src + (size_t)s * kSlotBytes, bytes, &sm.full[stage], pol_ef);
           else bulk_g2s(sm.ring + (size_t)stage * kSlotBytes, src + (size_t)s * kSlotBytes, bytes, &sm.full[stage]);
-          issued_bytes += bytes, ++issued;
           if (++stage == p.stages) stage = 0, par ^= 1;
         }
       }
-      if (!early_done) early(issued_bytes);
-      if (!p.pf_early) {
-        // own stream fully issued: pull the head of this CTA's region of the NEXT kernel's weights into L2, so HBM keeps
-        // streaming through our epilogue, the launch gap and the next kernel's prologue
-        if (p.next_w && p.next_bytes > 0)
-          prefetch_next_stream(p.next_w, p.next_bytes, p.next_tiles, p.next_grid, p.next_window, cta, n_cta);
-        // (the dependency has long resolved when the last weight slot is issued; the wait makes the pos read exact)
-        if (EPI == B200_EPI_QKV && p.prefetch_kv) kv_prefetch(true);
+      // own stream fully issued: pull the head of this CTA's region of the NEXT kernel's weights into L2, so HBM keeps
+      // streaming through our epilogue, the launch gap and the next kernel's prologue
+      if (p.next_w && p.next_bytes > 0)
+        prefetch_next_stream(p.next_w, p.next_bytes, p.next_tiles, p.next_grid, p.next_window, cta, n_cta);
+      if (EPI == B200_EPI_QKV && p.prefetch_kv) {
+        // the attention kernel that follows streams K/V rows [0, pos] of every kv head.  The dependency has long resolved
+        // when the last weight slot is issued; the wait makes the pos read exact.
+        pdl_wait();
+        const int kv_len = min(max(p.pos[0], 0) + 1, p.cache_seq);
+        const int brow = p.t_base / p.tokens_per_seq;
+        const uint32_t k_bytes = (uint32_t)kv_len * 256u, v_bytes = (uint32_t)((kv_len + 31) >> 5) * 8192u;
+        constexpr uint32_t piece = 16384;
+        const int kp = (int)((k_bytes + piece - 1) / piece), vp = (int)((v_bytes + piece - 1) / piece);
+        const int total = p.hkv * (kp + vp);
+#pragma unroll 1
+        for (int i = cta; i < total; i += n_cta) {
+          const int head = i / (kp + vp), j = i % (kp + vp);
+          const size_t base = ((size_t)brow * p.hkv + head) * p.cache_seq * 128;  // halfs, same for K and V
+          const bool k = j < kp;
+          const uint32_t off = (uint32_t)(k ? j : j - kp) * piece;
+          l2_prefetch(reinterpret_cast<const uint8_t*>((k ? p.kcache : p.vtcache) + base) + off, min(piece, (k ? k_bytes : v_bytes) - off));
+        }
       }
     }
     return;
@@ -163,11 +129,11 @@ __global__ void __launch_bounds__(kThreads, 1) gemv1_kernel(const __grid_constan
   }
   // griddepcontrol.wait happens inside the staging, after the constant loads (norm weight) have been issued
   G1State st;
-  g1_mma_phase<kDyn, GROUPED, true>(p, sm, warp, lane, cta, n_cta, st, /*wait_dep=*/true, x_ready);
+  g1_mma_phase<kDyn, GROUPED, true>(p, sm, warp, lane, cta, n_cta, st, /*wait_dep=*/true);
 }
 
 static size_t g1_smem_bytes(int stages, int xq_stride, bool grouped, int KB) {
-  size_t b = (size_t)stages * kSlotBytes + (size_t)stages * 16 + 6 * 8;
+  size_t b = (size_t)stages * kSlotBytes + (size_t)stages * 16 + 4 * 8;
   b += (size_t)2 * kConsumerWarps * 128 * 4;
   b += 32 * 4;
   b += (size_t)kPlanes * xq_stride;
@@ -249,15 +215,8 @@ int gemv1_launch(const b200_gemv_args_t* a, GemvParams p, cudaStream_t st) {
   p.next_window = prefetch_window_bytes();
   const int pf_kv = tune_get("B200_PF_KV", 1);
   p.prefetch_kv = (p.epi == B200_EPI_QKV && a->prefetch_kv && pf_kv) ? 1 : 0;
-  const int self_pf_kb = tune_get("B200_SELF_PF_KB", 0);
-  const int pf_early = tune_get("B200_PF_EARLY", 0);
-  p.self_pf_bytes = (a->prefetch_next || a->prefetch_kv) ? self_pf_kb * 1024 : 0;  // follows the engine's prefetch switch
-  p.pf_early = pf_early;
   p.keep_const = tune_get("B200_KEEP_CONST", 1);
-  p.hold_slots = tune_get("B200_G1_HOLD_SLOTS", 0);
-  p.warm = tune_get("B200_G1_WARM", 0);  // measured: the cold pass takes longer than the dependency wait it was meant to fill
   p.stream_ef = tune_get("B200_STREAM_EF", 1);
-  p.dbg = tune_get("B200_G1_DBG", 0);
   p.const_pf = tune_get("B200_CONST_PF", 1) ? static_cast<const uint8_t*>(a->prefetch_const) : nullptr;
   p.const_pf_bytes = a->prefetch_const_bytes;
   const int grid = std::min(p.n_tiles, sm_count());

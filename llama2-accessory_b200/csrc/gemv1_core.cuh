@@ -99,57 +99,81 @@ __device__ __forceinline__ float stage_piece(const uint4& xo, uint8_t* xq, int x
   return hsum8(xo);
 }
 
-// dry = instruction-cache warm-up pass (stand-alone kernel only): the same instructions run once BEFORE the dependency on the
-// previous kernel resolves, with every global access and stamp switched off (shared-memory results are overwritten by the
-// real pass), so that the real pass -- which sits on the critical path of the launch -- does not stall on instruction fetch.
+// Timeline stamps (b200_timeline / b200_timeline_cta) are off unless a profiling run asks for them: the work sits out of
+// line, so that the straight-line code between the dependency wait and the first MMA stays short.  i >= 8: per-CTA only.
+static __device__ __noinline__ void g1_stamp_cold(unsigned long long* tl, unsigned long long* tlc, int cta, int i) {
+  if (i < 8) tl_max(tl, i);
+  tl_cta(tlc, cta, i);
+}
+__device__ __forceinline__ void g1_stamp(const GemvParams& p, int cta, int i, bool me = threadIdx.x == 0) {
+  if (me && (p.tl || p.tlc)) g1_stamp_cold(p.tl, p.tlc, cta, i);
+}
+
+// residual delta of 8 elements: a plain fp16 vector at TP = 1; the sum over tensor-parallel ranks (plain or LL buffers,
+// load_delta8) runs out of line.  Scalar arguments: a reference to the caller's parameter block would move it to local memory.
+static __device__ __noinline__ uint4 g1_delta8_ranks(const __half* delta, int K, int n_delta, int ll_in, const unsigned* ll_step,
+                                                     int ll_period, int ll_in_id, unsigned* ll_err, int off) {
+  GemvParams q;
+  q.delta = delta, q.K = K, q.n_delta = n_delta, q.ll_in = ll_in, q.ll_step = ll_step, q.ll_period = ll_period;
+  q.ll_in_id = ll_in_id, q.ll_err = ll_err;
+  return load_delta8(q, (size_t)off);
+}
+__device__ __forceinline__ uint4 g1_delta8(const GemvParams& p, int off) {
+  if (!p.ll_in && p.n_delta <= 1) return ldg_cg_v4(p.delta + off);
+  return g1_delta8_ranks(p.delta, p.K, p.n_delta, p.ll_in, p.ll_step, p.ll_period, p.ll_in_id, p.ll_err, off);
+}
+
 template <int PRO_T, bool GROUPED = false>
-__device__ __forceinline__ float stage_own_slice_pass(const GemvParams& p, const G1Smem& sm, int xq_stride, int warp, int lane,
-                                                      int slots_per_tile, int cta, bool wait_dep, bool dry) {
+__device__ __forceinline__ float stage_own_slice(const GemvParams& p, const G1Smem& sm, int xq_stride, int warp, int lane,
+                                                 int slots_per_tile, int cta, bool wait_dep = false) {
   const int PRO = PRO_T == kDyn ? p.pro : PRO_T;
   // lane -> (slot parity, block of the warp's pair, 8-element piece): one 16-byte load covers 8 elements
   const int half = lane >> 4, sub = lane & 15;
   const int n_it = (slots_per_tile + 1) >> 1;
   float xs = 0.f;
-  constexpr int kMaxIt = 2;  // RMSNorm: K <= 8192 -> <= 4 slots per tile
-  uint4 hv[kMaxIt], gv[kMaxIt];
-  bool ok[kMaxIt];
-  int e0s[kMaxIt];
+  // every load of the slice is in flight before the first conversion (K = 11008: 3 pieces per lane; a dependent
+  // load -> convert -> store loop would pay one loaded L2 round trip per piece).  RMSNorm: xv = the residual sums.
+  constexpr int kMaxPieces = 4;  // K <= 16384
+  constexpr int kMaxIt = 2;      // RMSNorm: K <= 8192 -> <= 4 slots per tile
+  uint4 xv[kMaxPieces], gv[kMaxIt];
+#pragma unroll
+  for (int it = 0; it < kMaxPieces; ++it) xv[it] = make_uint4(0, 0, 0, 0);
   float rstd = 1.f;
   if (PRO == B200_PRO_RMSNORM) {
     float ssq = 0.f;
+    bool ok[kMaxIt];
+    int e0s[kMaxIt];
 #pragma unroll
     for (int it = 0; it < kMaxIt; ++it) {  // the norm weight is a constant: requested before the dependency resolves
       const int s = 2 * it + half;
       const int blk = s * kSlotBlocks + warp * kChunk + (sub >> 3);
       ok[it] = it < n_it && s < slots_per_tile && blk < p.KB;
       e0s[it] = blk * 64 + (sub & 7) * 8;
-      hv[it] = gv[it] = make_uint4(0, 0, 0, 0);
-      if (ok[it] && !dry) {
-        if (p.dbg == 3) gv[it] = make_uint4(0x3c003c00u, 0x3c003c00u, 0x3c003c00u, 0x3c003c00u);  // measurement knob: gamma = 1, no load
-        else gv[it] = p.keep_const ? ldg_keep_v4(p.gamma + e0s[it], l2_policy_evict_last()) : *reinterpret_cast<const uint4*>(p.gamma + e0s[it]);
-      }
+      gv[it] = make_uint4(0, 0, 0, 0);
+      if (ok[it]) gv[it] = p.keep_const ? ldg_keep_v4(p.gamma + e0s[it], l2_policy_evict_last()) : *reinterpret_cast<const uint4*>(p.gamma + e0s[it]);
     }
-    if (wait_dep && !dry) pdl_wait();
-    if (threadIdx.x == 0 && !dry) tl_max(p.tl, 4), tl_cta(p.tlc, cta, 4);
+    if (wait_dep) pdl_wait();
+    g1_stamp(p, cta, 4);
 #pragma unroll
-    for (int it = 0; it < kMaxIt; ++it) {
-      if (ok[it] && !dry) {
-        uint4 a = ldg_cg_v4(p.resid + e0s[it]);  // L2-coherent: in the persistent kernel another CTA wrote it this launch
-        if (p.delta && p.dbg != 4) {
-          const uint4 b = load_delta8(p, (size_t)e0s[it]);
-          __half2* ha = reinterpret_cast<__half2*>(&a);
-          const __half2* hb = reinterpret_cast<const __half2*>(&b);
+    for (int it = 0; it < kMaxIt; ++it)
+      if (ok[it]) xv[it] = ldg_cg_v4(p.resid + e0s[it]);  // L2-coherent: in the persistent kernel another CTA wrote it this launch
+    if (p.delta) {
+      uint4 dv[kMaxIt];
 #pragma unroll
-          for (int j = 0; j < 4; ++j) ha[j] = __hadd2(ha[j], hb[j]);  // the reference's fp16 residual add
-        }
-        hv[it] = a;
+      for (int it = 0; it < kMaxIt; ++it) dv[it] = ok[it] ? g1_delta8(p, e0s[it]) : make_uint4(0, 0, 0, 0);
+#pragma unroll
+      for (int it = 0; it < kMaxIt; ++it) {
+        __half2* ha = reinterpret_cast<__half2*>(&xv[it]);
+        const __half2* hb = reinterpret_cast<const __half2*>(&dv[it]);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) ha[j] = __hadd2(ha[j], hb[j]);  // the reference's fp16 residual add
       }
     }
 #pragma unroll
     for (int it = 0; it < kMaxIt; ++it) {
       if (ok[it]) {
-        if (p.h_out && cta == 0 && !dry) *reinterpret_cast<uint4*>(p.h_out + e0s[it]) = hv[it];
-        const __half2* h = reinterpret_cast<const __half2*>(&hv[it]);
+        if (p.h_out && cta == 0) *reinterpret_cast<uint4*>(p.h_out + e0s[it]) = xv[it];
+        const __half2* h = reinterpret_cast<const __half2*>(&xv[it]);
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const float2 f = __half22float2(h[j]);
@@ -159,28 +183,22 @@ __device__ __forceinline__ float stage_own_slice_pass(const GemvParams& p, const
       }
     }
     ssq = warp_sum(ssq);
-    if (threadIdx.x == 0 && !dry) tl_cta(p.tlc, cta, 8);
+    g1_stamp(p, cta, 8);
     if (lane == 0) sm.scratch[warp] = ssq;
     named_bar_sync(1, kConsumerThreads);
-    if (threadIdx.x == 0 && !dry) tl_cta(p.tlc, cta, 9);
+    g1_stamp(p, cta, 9);
     float tot = 0.f;
 #pragma unroll
     for (int wi = 0; wi < kConsumerWarps; ++wi) tot += sm.scratch[wi];
     rstd = 1.0f / sqrtf(tot / (float)p.K + p.eps);
   }
-  // every load of the slice is in flight before the first conversion (K = 11008: 3 pieces per lane; a dependent
-  // load -> convert -> store loop would pay one loaded L2 round trip per piece)
-  constexpr int kMaxPieces = 4;  // K <= 16384
-  uint4 xv[kMaxPieces];
-  if (PRO != B200_PRO_RMSNORM && wait_dep && !dry) pdl_wait();
+  if (PRO != B200_PRO_RMSNORM && wait_dep) pdl_wait();
   if (PRO == B200_PRO_NONE) {
 #pragma unroll
     for (int it = 0; it < kMaxPieces; ++it) {
       const int s = 2 * it + half;
       const int blk = s * kSlotBlocks + warp * kChunk + (sub >> 3);
-      xv[it] = make_uint4(0, 0, 0, 0);
-      if (it < n_it && s < slots_per_tile && blk < p.KB && !dry)
-        xv[it] = ldg_cg_v4(p.xin + blk * 64 + (sub & 7) * 8);
+      if (it < n_it && s < slots_per_tile && blk < p.KB) xv[it] = ldg_cg_v4(p.xin + blk * 64 + (sub & 7) * 8);
     }
   }
   if (PRO_T == kProAttnMerge) {
@@ -194,7 +212,6 @@ __device__ __forceinline__ float stage_own_slice_pass(const GemvParams& p, const
     for (int it = 0; it < kMaxPieces; ++it) {
       const int s = 2 * it + half;
       const int blk = s * kSlotBlocks + warp * kChunk + (sub >> 3);
-      xv[it] = make_uint4(0, 0, 0, 0);
       if (it < n_it && s < slots_per_tile && blk < p.KB) {
         const int e0 = blk * 64 + (sub & 7) * 8, hq = e0 >> 7, d0 = e0 & 127;
         constexpr int kMaxSplit = 8;
@@ -229,27 +246,27 @@ __device__ __forceinline__ float stage_own_slice_pass(const GemvParams& p, const
       }
     }
   }
-#pragma unroll
-  for (int it = 0; it < kMaxPieces; ++it) {
+  // conversion, RMSNorm scaling, digit split and plane stores: ONE copy of the code, rolled over the pieces (the piece is
+  // picked from the loaded registers by a select chain, nothing goes through local memory); xs sums in piece order
+#pragma unroll 1
+  for (int it = 0; it < n_it; ++it) {
     const int s = 2 * it + half;
     const int blk = s * kSlotBlocks + warp * kChunk + (sub >> 3);
-    const bool valid = it < n_it && s < slots_per_tile && blk < p.KB;
+    const bool valid = s < slots_per_tile && blk < p.KB;
     const int e0 = blk * 64 + (sub & 7) * 8;
-    uint4 xo = make_uint4(0, 0, 0, 0);
+    uint4 xo = xv[0];
+#pragma unroll
+    for (int j = 1; j < kMaxPieces; ++j) xo = it == j ? xv[j] : xo;
     if (valid) {
       if (PRO == B200_PRO_RMSNORM) {
         const uint4 gm = it == 0 ? gv[0] : gv[1];
-        const uint4 hvi = it == 0 ? hv[0] : hv[1];
-        const __half2* h = reinterpret_cast<const __half2*>(&hvi);
         const __half2* gh = reinterpret_cast<const __half2*>(&gm);
         __half2* o = reinterpret_cast<__half2*>(&xo);
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          const float2 f = __half22float2(h[j]);
+          const float2 f = __half22float2(o[j]);
           o[j] = __hmul2(__floats2half2_rn(f.x * rstd, f.y * rstd), gh[j]);  // components.py:52-53 rounding points
         }
-      } else {
-        xo = xv[it];
       }
       xs += hsum8(xo);
       uint32_t lo[kPlanes], hi[kPlanes];
@@ -268,17 +285,6 @@ __device__ __forceinline__ float stage_own_slice_pass(const GemvParams& p, const
   }
   xs = warp_sum(xs);
   __syncwarp();
-  return xs;
-}
-
-template <int PRO_T, bool GROUPED = false>
-__device__ __forceinline__ float stage_own_slice(const GemvParams& p, const G1Smem& sm, int xq_stride, int warp, int lane,
-                                                 int slots_per_tile, int cta, bool wait_dep = false) {
-  float xs = 0.f;
-  const int first = (PRO_T == kDyn && wait_dep && p.warm) ? 0 : 1;
-#pragma unroll 1
-  for (int pass = first; pass < 2; ++pass)
-    xs = stage_own_slice_pass<PRO_T, GROUPED>(p, sm, xq_stride, warp, lane, slots_per_tile, cta, wait_dep, pass == 0);
   return xs;
 }
 
@@ -318,7 +324,7 @@ __device__ __forceinline__ void g1_mma_tiles(const GemvParams& p, const G1Smem& 
         for (int i = 0; i < 4; ++i) acc[c][k][i] = 0;
     for (int s = 0; s < slots_per_tile; ++s) {
       mbar_wait(&sm.full[stage], par);
-      if (p.tl && threadIdx.x == 0 && tile == tile_begin && s == 0) tl_max(p.tl, 7), tl_cta(p.tlc, cta, 7);
+      if (tile == tile_begin && s == 0) g1_stamp(p, cta, 7);
       const uint32_t wa = ring32 + (uint32_t)stage * kSlotBytes;
       const int blk0 = s * kSlotBlocks + warp * kChunk;
       if (GROUPED) {
@@ -442,10 +448,8 @@ __device__ __forceinline__ void g1_mma_tiles(const GemvParams& p, const G1Smem& 
     if (lane == 0) mbar_arrive(&sm.red_full[buf]);
   }
   st.stage = stage, st.par = par, st.lt = lt;
-  if (threadIdx.x == 0) {
-    tl_max(p.tl, 2), tl_cta(p.tlc, cta, 2);
-    if (p.tlc) p.tlc[(size_t)cta * 16 + 5] = (unsigned long long)(tile_end - tile_begin);
-  }
+  g1_stamp(p, cta, 2);
+  if (threadIdx.x == 0 && p.tlc) p.tlc[(size_t)cta * 16 + 5] = (unsigned long long)(tile_end - tile_begin);
 }
 
 
@@ -453,12 +457,11 @@ __device__ __forceinline__ void g1_mma_tiles(const GemvParams& p, const G1Smem& 
 // (griddepcontrol.wait / grid barrier) before the call.
 template <int PRO_T, bool GROUPED = false, bool ARED = false>
 __device__ __forceinline__ void g1_mma_phase(const GemvParams& p, const G1Smem& sm, int warp, int lane, int cta, int n_cta,
-                                             G1State& st, bool wait_dep = false, uint64_t* x_ready = nullptr) {
+                                             G1State& st, bool wait_dep = false) {
   const int slots_per_tile = (p.KB + kSlotBlocks - 1) / kSlotBlocks;
   const int xq_stride = (((p.K + 127) >> 7) << 7) + 64;  // plane stride = 64 mod 128: planes g, g+1 hit different banks
   const float xs_w = stage_own_slice<PRO_T, GROUPED>(p, sm, xq_stride, warp, lane, slots_per_tile, cta, wait_dep);
-  if (x_ready && lane == 0) mbar_arrive(x_ready);
-  if (threadIdx.x == 0) tl_max(p.tl, 1), tl_cta(p.tlc, cta, 1);
+  g1_stamp(p, cta, 1);
 
   g1_mma_tiles<GROUPED, ARED>(p, sm, warp, lane, cta, n_cta, st, xs_w);
 }
@@ -504,6 +507,7 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
   // the scales are constants: their round trip overlaps the wait for the previous kernel (stand-alone launch)
   if (staged && !GROUPED) {
     const uint64_t pol = l2_policy_evict_last();
+#pragma unroll 1
     for (int i = etid; i < n_local * 16; i += kEpiWarps * 32)
       sz_s[i] = p.keep_const ? h2bits(ldg_keep_u32(&p.sz[(size_t)tile_begin * 16 + i], pol)) : p.sz[(size_t)tile_begin * 16 + i];
   }
@@ -512,6 +516,7 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
   if (EPI == B200_EPI_QKV) ps = p.pos[0];
   if (staged) {
     if (EPI == B200_EPI_QKV)
+#pragma unroll 1
       for (int i = etid; i < n_local * 16; i += kEpiWarps * 32) {
         const int row = tile_begin * 16 + i;
         const bool rot = row < p.n_q_rows + p.n_kv_rows;
@@ -520,7 +525,7 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
       }
     asm volatile("bar.sync 2, %0;" ::"n"(kEpiWarps * 32) : "memory");
   }
-  if (etid == 0) tl_max(p.tl, 6), tl_cta(p.tlc, cta, 6);
+  g1_stamp(p, cta, 6, etid == 0);
   const int c = etid & 7, r0 = etid >> 3;
   // weight of plane c: digits are in units of 2^(7c-24), the hand-off carries 16 x the sum
   const float pw = c < kPlanes ? __int_as_float((127 + 7 * c - 28) << 23) : 0.f;
@@ -536,15 +541,23 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
         sza = p.sz[(size_t)tile * 16 + r0], szb = p.sz[(size_t)tile * 16 + r0 + 8];
       }
     }
+    // QKV: the q | k | v boundaries are multiples of the 128-row head, so a 16-row tile lies in one head of one of them;
+    // its class, the head offset d0 of row 0 and its destination are decided once per tile
     float2 cs[2];
+    int kind = 0, d0 = 0;  // kind: 0 = q, 1 = k, 2 = v
+    __half* dst = nullptr;
     if (EPI == B200_EPI_QKV) {
+      const int row0 = tile * 16;
+      kind = row0 < p.n_q_rows ? 0 : (row0 < p.n_q_rows + p.n_kv_rows ? 1 : 2);
+      const int local0 = row0 - (kind == 0 ? 0 : (kind == 1 ? p.n_q_rows : p.n_q_rows + p.n_kv_rows));
+      d0 = local0 & 127;
+      const size_t hbase = ((size_t)(p.t_base / p.tokens_per_seq) * p.hkv + (local0 >> 7)) * p.cache_seq * 128;
+      dst = kind == 0 ? reinterpret_cast<__half*>(p.out) + row0
+                      : (kind == 1 ? p.kcache + hbase + (size_t)ps * 128 : p.vtcache + hbase + (size_t)(ps >> 5) * 4096 + (ps & 31));
+      const float2* rope_row = p.rope + (size_t)ps * 64;
 #pragma unroll
-      for (int hh = 0; hh < 2; ++hh) {
-        const int row = tile * 16 + r0 + 8 * hh;
-        const bool rot = row < p.n_q_rows + p.n_kv_rows;
-        const int d = (row < p.n_q_rows ? row : row - p.n_q_rows) & 127;
-        cs[hh] = staged ? rope_s[li * 16 + r0 + 8 * hh] : (rot ? p.rope[(size_t)ps * 64 + (d >> 1)] : make_float2(1.f, 0.f));
-      }
+      for (int hh = 0; hh < 2; ++hh)
+        cs[hh] = kind == 2 ? make_float2(1.f, 0.f) : (staged ? rope_s[li * 16 + r0 + 8 * hh] : rope_row[(d0 + r0 + 8 * hh) >> 1]);
     }
     mbar_wait(&sm.red_full[buf], (lt >> 1) & 1);
     const int* rbase = sm.red + (size_t)buf * kConsumerWarps * 128;
@@ -623,11 +636,13 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
             if (c == 0 && (r0 & 1) == 0) {
               const unsigned pay = (unsigned)__half_as_ushort(y16) | (other << 16);
               const unsigned seq = *p.ll_step * (unsigned)p.ll_period + (unsigned)p.ll_out_id + 1u;
+#pragma unroll 1
               for (int rr = 0; rr < p.n_bcast; ++rr)
                 ll::ll_store(reinterpret_cast<uint8_t*>(p.bcast[rr]) + (size_t)(p.bcast_off + row) * 4, pay, seq);
             }
           } else if (c == 0) {
             if (p.n_bcast > 0) {  // row-parallel partial sums: pushed into every rank's buffer (the all-reduce's data movement)
+#pragma unroll 1
               for (int rr = 0; rr < p.n_bcast; ++rr) reinterpret_cast<__half*>(p.bcast[rr])[p.bcast_off + row] = y16;
             } else {
               reinterpret_cast<__half*>(p.out)[row] = y16;
@@ -638,12 +653,8 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
         } else {  // B200_EPI_QKV
           const float mine = __half2float(y16);
           const float other = __shfl_xor_sync(0xffffffffu, mine, 8);  // row r^1
-          const int brow = p.t_base / p.tokens_per_seq;
-          const bool is_v = row >= p.n_q_rows + p.n_kv_rows;
-          const int local = row < p.n_q_rows ? row : (is_v ? row - p.n_q_rows - p.n_kv_rows : row - p.n_q_rows);
-          const int head = local >> 7, d = local & 127;
           float val = mine;
-          if (!is_v) {
+          if (kind != 2) {
             // interleaved-pair complex rotation in fp32 (llama.py:67-77), no FMA contraction
             const float xe = (r & 1) ? other : mine, xo = (r & 1) ? mine : other;
             val = (r & 1) ? __fadd_rn(__fmul_rn(xe, cs[hh].y), __fmul_rn(xo, cs[hh].x))
@@ -651,20 +662,17 @@ __device__ __forceinline__ void g1_epilogue_phase(const GemvParams& p, const G1S
           }
           const __half o16 = __float2half_rn(val);
           if (c == 0) {
-            if (row < p.n_q_rows) {
-              reinterpret_cast<__half*>(p.out)[row] = o16;
-            } else if (!is_v) {
-              p.kcache[(((size_t)brow * p.hkv + head) * p.cache_seq + ps) * 128 + ((((d >> 3) ^ ((ps & 1) << 2)) << 3) | (d & 7))] = o16;
-            } else {
-              p.vtcache[((size_t)brow * p.hkv + head) * p.cache_seq * 128 + (size_t)(ps >> 5) * 4096 + d * 32 + (ps & 31)] = o16;
-            }
+            const int d = d0 + r;
+            if (kind == 0) dst[r] = o16;
+            else if (kind == 1) dst[(((d >> 3) ^ ((ps & 1) << 2)) << 3) | (d & 7)] = o16;
+            else dst[d * 32] = o16;
           }
         }
       }
     }
   }
   lt_io = lt;
-  if (etid == 0) tl_max(p.tl, 3), tl_cta(p.tlc, cta, 3);
+  g1_stamp(p, cta, 3, etid == 0);
 }
 
 }  // namespace b200

@@ -67,14 +67,8 @@ struct GemvParams {
   int stages, x_stride, n_chunk64;
   const uint8_t* next_w;  // the NEXT kernel's weight stream; region heads are prefetched into L2 by the producer
   int next_bytes, next_tiles, next_grid, next_window;
-  int prefetch_kv;  // QKV epilogue: also pull the K/V rows the following attention kernel reads into L2 (2: at ring-full time)
-  // gemv1.cu: bytes of this CTA's OWN region beyond the ring that the producer prefetches into L2 as soon as the ring is
-  // full (HBM keeps streaming while the consumers still wait for the previous kernel), and whether the next-stream /
-  // K-V prefetches are issued at that point too instead of after the last own slot
-  int self_pf_bytes, pf_early;
+  int prefetch_kv;  // QKV launch: the producer also pulls the K/V rows the following attention kernel reads into L2
   int stream_ef;               // weight bulk copies carry the L2 evict_first policy (B200_STREAM_EF)
-  int warm;                    // gemv1: instruction-cache warm-up pass of the activation staging before the dependency wait (B200_G1_WARM)
-  int hold_slots;              // gemv1 experiment: producer pauses after this many slots until x is staged (0 = off)
   int keep_const;              // norm weight / scales loaded with the L2 evict_last hint (B200_KEEP_CONST)
   const uint8_t* const_pf;     // a later kernel's small constants (its norm weight): CTA 0 prefetches them into L2 first thing
   int const_pf_bytes;

@@ -30,7 +30,7 @@ tl = torch.zeros((NROW, 8), dtype=torch.int64, device="cuda")
 tlc = torch.zeros((NL, NCTA, 16), dtype=torch.int64, device="cuda")
 def run(ks):
     for k in ALL_KNOBS:
-        lib.b200_tune(k.encode(), -1 if k not in ("B200_G1_DBG", "B200_G1_HOLD_SLOTS") else 0)
+        lib.b200_tune(k.encode(), -1)
     defaults = {"B200_PF_KB": 96, "B200_PF_KV": 1, "B200_G1_ARED": 1, "B200_KEEP_CONST": 1, "B200_CONST_PF": 1, "B200_ATTN_EVEN": 1}
     for k in ALL_KNOBS:
         if k in defaults:
